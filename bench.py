@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--mode fwd|train] [--batch 256] [--precision fp16x3|fp32]
     python bench.py --impl reference ...     # the reference algorithm on the host cores (oracle port)
     python bench.py --elide-padding 0|1|2    # ablation of the padding-vertex elision (default: library default = 1)
+    python bench.py --dump-outputs DIR       # also write the last timed step's outputs as DIR/<name>.npy
     torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): batch 256 synthetic H36M 17-joint poses [256,17,5] ~ N(0,1),
@@ -61,7 +62,30 @@ def parse():
     ap.add_argument("--mesh", default="smpl", choices=["smpl", "mano"],
                     help="smpl: 6890-vertex SMPL-size hierarchy (default, BASELINE configs[1,2,4]); "
                          "mano: 778-vertex MANO-size hierarchy 1088..68, 21 joints (configs[3], use --batch 1024)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (fwd: the meshes; "
+                         "train: the loss and every parameter's gradient); at most 64 MB in all")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one .npy per output array, float32 as computed.  The inputs are seeded, so two builds run with
+    the same arguments can be compared file by file.  Above DUMP_BYTES in all, every array keeps the same share of its
+    leading-axis rows (e.g. whole meshes), picked by a fixed seed."""
+    os.makedirs(path, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    keep = min(1.0, DUMP_BYTES / max(total, 1))
+    rng = np.random.default_rng(0)
+    for name, a in arrays.items():
+        if keep < 1.0 and a.ndim > 0:
+            a = a[np.sort(rng.choice(a.shape[0], max(1, int(a.shape[0] * keep)), replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -253,10 +277,11 @@ def capture_stdout():
     os.dup2(2, 1)
 
 
-def measure_train(model, x_host, dev, B, world, rank, steps, warmup, flush, barrier):
+def measure_train(model, x_host, dev, B, world, rank, steps, warmup, flush, barrier, outputs=None):
     """configs[2]/[4]: forward + backward (L1 loss to random targets, train-mode BatchNorm, B per GPU) + the single
     all-reduce of the flat gradient.  Device-timed per step (CUDA events), max over ranks; the all-reduce is also
-    timed on its own (events around the collective: it runs after backward on the same stream, i.e. fully exposed)."""
+    timed on its own (events around the collective: it runs after backward on the same stream, i.e. fully exposed).
+    If `outputs` is a dict, it receives the last timed step's loss and reduced gradients (host float32 arrays)."""
     import torch.distributed as dist
 
     from pose2mesh_release_b200.dist import DataParallelStep
@@ -287,10 +312,13 @@ def measure_train(model, x_host, dev, B, world, rank, steps, warmup, flush, barr
     for i in range(steps):
         flush.zero_()
         evs[i][0].record()
-        launch(evs[i][2:])
+        loss = launch(evs[i][2:])
         evs[i][1].record()
     barrier()
     launches = int(_lib.load().p2m_launch_count())
+    if outputs is not None:
+        outputs["loss"] = loss.detach().float().cpu().numpy()
+        outputs.update({"grad." + k: p.grad.detach().float().cpu().numpy() for k, p in model.named_parameters()})
     step_ms = sum(e[0].elapsed_time(e[1]) for e in evs)
     ar_ms = sum(e[2].elapsed_time(e[3]) for e in evs)
     t = torch.tensor([step_ms, ar_ms], device=dev, dtype=torch.float64)
@@ -374,7 +402,8 @@ def main():
         if rank == 0:
             sampler.start()
             sampler.mark()
-        tr = measure_train(model, x_host, dev, B, world, rank, args.steps, args.warmup, flush, barrier)
+        outputs = {} if args.dump_outputs and rank == 0 else None
+        tr = measure_train(model, x_host, dev, B, world, rank, args.steps, args.warmup, flush, barrier, outputs)
         clocks = sampler.stop() if rank == 0 else None
         if rank == 0:
             emit({"metric": "SMPL meshes/sec (fwd+bwd train step)", "value": tr["value"], "unit": "meshes/s", "n_gpus": world,
@@ -390,6 +419,8 @@ def main():
                              "l2": "256 MiB buffer written between timed iterations (outside the event pairs)"},
                   "e2e": tr["e2e"], "gpu_launches": tr["gpu_launches"], "gpu_launches_per_step": tr["gpu_launches_per_step"],
                   "clocks": clocks, "train": tr})
+            if outputs is not None:
+                dump_outputs(args.dump_outputs, outputs)
         if world > 1:
             dist.barrier()
             dist.destroy_process_group()
@@ -402,7 +433,7 @@ def main():
         with torch.no_grad():
             return model(x)
 
-    launch = step
+    launch, y_static = step, None
     if not args.no_graph:
         # replay the ~100-launch forward from a CUDA graph (the library only enqueues on the current stream)
         try:
@@ -412,7 +443,7 @@ def main():
             torch.cuda.synchronize()
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                y_static = step()  # noqa: F841  (keeps the graph's output alive)
+                y_static = step()  # the graph's output tensor: every replay rewrites it
             torch.cuda.synchronize()
             step_graph, launch = graph, graph.replay
         except Exception as e:  # keep the bench alive; say so in the JSON
@@ -434,11 +465,14 @@ def main():
     for i in range(args.steps):
         flush.zero_()               # evict L2 between timed iterations (not timed)
         evs[i][0].record()
-        launch()
+        y_last = launch()
         evs[i][1].record()
     barrier()
     launches_eager = lib.p2m_launch_count()
     clocks = sampler.stop() if rank == 0 else None
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        outputs = {"meshes": (y_static if step_graph is not None else y_last).float().cpu().numpy()}
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     t = torch.tensor([total_ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -563,6 +597,8 @@ def main():
             "clocks": clocks, "roofline": roofline, "cpu_baseline": cpu_baseline, "train": train, "layers": layers,
         }
         emit(line)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

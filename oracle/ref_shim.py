@@ -11,10 +11,9 @@ in-process, with the three shims SURVEY.md §8(c) lists:
   3. ``torch.Tensor.cuda`` -> identity while the reference runs on CPU
      (lib/models/meshnet.py:81 hard-codes .cuda()).
 
-/root/reference exists only in the build container, never on the GPU box, so this
-module is used exclusively by tests/golden/make_golden.py (fixture generation) and by
-CPU tests that are skipped when the tree is absent.  Nothing in the product path,
-``-m gpu`` tests, smoke() or bench.py imports it.
+The reference tree is not part of this repository, so this module is used exclusively by
+the fixture generators tests/golden/make_golden*.py; the tests compare with the fixtures
+they wrote.  Nothing in the product path, the tests, smoke() or bench.py imports it.
 """
 import contextlib
 import os

@@ -62,9 +62,6 @@ def _train_step_parity(name, n_distinct, copies, open_relus, precision="fp16x3")
     tgt = td.repeat(copies, 1, 1).to(dev())
     y = model(x)
     loss = (y - tgt).abs().mean()
-    loss.backward()
-    torch.cuda.synchronize()
-    assert model._hier.kernel_status(torch.cuda.current_device()) == 0
     del tgt
 
     sd_o = {k: (v.clone().requires_grad_(True) if v.is_floating_point() and "running" not in k else v.clone())
@@ -73,6 +70,13 @@ def _train_step_parity(name, n_distinct, copies, open_relus, precision="fp16x3")
     yo = mo.forward(sd_o, laps, xo, mano=mano, training=True)
     lo = (yo - td).abs().mean()
     lo.backward()
+    # Both backward passes start from the same dL/dy, the oracle's sign(yo - td) / N.  The L1 loss has a kink at
+    # y == tgt that open ReLUs do not hold open: of the B * V * 3 outputs, one can lie within the two fp32
+    # implementations' difference of its target, flip sign, and move that mesh's dx by O(1e-3) of max |dx| (seen on
+    # one host and not on another: |yo - td| = 4e-6 at 1 of 1.2 M entries, dx off by 1.8e-3 there, 7e-5 elsewhere).
+    y.backward((torch.sign(yo.detach() - td).repeat(copies, 1, 1) / y.numel()).to(dev()))
+    torch.cuda.synchronize()
+    assert model._hier.kernel_status(torch.cuda.current_device()) == 0
 
     y_cpu = y.detach().cpu()
     assert y_cpu.shape == (B, v0, 3)
