@@ -226,6 +226,19 @@ int p2m_regress_joints(const float* joint_regressor, const float* vertices, floa
 int p2m_normalize_pose2d(const float* joints_px, float* pose2d, int batch, int n_joint, int input_h, int input_w,
                          int truncate_like_int_input, p2m_stream_t stream);
 
+/* ---- the demo's camera fit (SURVEY.md §8 row f5; demo/run.py:149-189, lib/models/project_net.py) --------------
+ * The projection target: joints_px [B, J, 2] (J <= 32) -> out_px [B, J, 2], the joints in pixels of a res_w x res_h
+ * patch cut around the box process_bbox(get_bbox(joints), aspect_ratio, scale) (the demo: 500 x 500, 1.0, 1.25), and
+ * out_bbox [B, 4] = that box [x, y, w, h] (the demo's bbox1).  truncate_like_int_input as in p2m_normalize_pose2d.   */
+int p2m_crop_pose2d(const float* joints_px, float* out_px, float* out_bbox, int batch, int n_joint, int res_w, int res_h,
+                    float aspect_ratio, float scale, int truncate_like_int_input, p2m_stream_t stream);
+/* The weak-perspective camera out = (p[:, :2] + c[1:]) * c[0] * crop_size / 2 + crop_size / 2 fitted per person to
+ * target_px [B, J, 2] by `iters` steps of mean L1 loss + Adam (torch.optim.Adam defaults; lr 0.1, 0.05 from step 502,
+ * 0.001 from step 1002), starting from cam_init [B, 3].  joints3d [B, J, joint_stride] (x, y first; joint_stride >= 2),
+ * J <= 32.  Writes cam_out [B, 3] and loss_out [B], the L1 loss of the final camera.  One warp per person.          */
+int p2m_fit_camera(const float* joints3d, const float* target_px, const float* cam_init, float* cam_out, float* loss_out,
+                   int batch, int n_joint, int joint_stride, double crop_size, int iters, p2m_stream_t stream);
+
 /* ---- the mesh losses (SURVEY.md §8 row f3; lib/core/loss.py:10-23,62-114) ---------------------------
  * One pass over (mesh, face): sums[0] = sum of the NormalVectorLoss terms, sums[1] = sum of the EdgeLengthLoss terms
  * over (B, 3 n_face) (fp64, device; the losses are sums / (3 B n_face)).  If grad_out [B, n_vertex, 3] is given it

@@ -97,7 +97,7 @@ EXPORTS = [
     "p2m_model_create", "p2m_model_destroy", "p2m_model_num_layers", "p2m_model_layer_info",
     "p2m_model_set_precision", "p2m_debug_kernel_status", "p2m_debug_set_trace", "p2m_debug_set_split_t1", "p2m_debug_set_fuse_head", "p2m_debug_set_elide_padding", "p2m_debug_set_dedup_padding", "p2m_debug_set_dw_swap", "p2m_model_set_profiling", "p2m_model_layer_times_ms", "p2m_meshnet_workspace_bytes", "p2m_meshnet_backward_scratch_bytes",
     "p2m_meshnet_forward", "p2m_meshnet_backward", "p2m_model_set_output_gather", "p2m_meshnet_forward_vertices", "p2m_meshnet_host_io_bytes", "p2m_meshnet_forward_host", "p2m_meshnet_forward_vertices_host",
-    "p2m_cheb_conv_workspace_bytes", "p2m_cheb_conv_fwd", "p2m_cheb_conv_bwd", "p2m_graph_match_level", "p2m_posenet_workspace_bytes", "p2m_posenet_forward", "p2m_regress_joints", "p2m_normalize_pose2d", "p2m_mesh_losses", "p2m_coord_loss",
+    "p2m_cheb_conv_workspace_bytes", "p2m_cheb_conv_fwd", "p2m_cheb_conv_bwd", "p2m_graph_match_level", "p2m_posenet_workspace_bytes", "p2m_posenet_forward", "p2m_regress_joints", "p2m_normalize_pose2d", "p2m_crop_pose2d", "p2m_fit_camera", "p2m_mesh_losses", "p2m_coord_loss",
     "p2m_last_error", "p2m_version", "p2m_launch_count", "p2m_launch_count_reset",
 ]
 
@@ -180,6 +180,11 @@ def load() -> C.CDLL:
         lib.p2m_regress_joints.restype = C.c_int
         lib.p2m_normalize_pose2d.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]
         lib.p2m_normalize_pose2d.restype = C.c_int
+        lib.p2m_crop_pose2d.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int,
+                                        vp]
+        lib.p2m_crop_pose2d.restype = C.c_int
+        lib.p2m_fit_camera.argtypes = [vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, vp]
+        lib.p2m_fit_camera.restype = C.c_int
         lib.p2m_mesh_losses.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp]
         lib.p2m_mesh_losses.restype = C.c_int
         lib.p2m_coord_loss.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp]

@@ -1498,14 +1498,16 @@ __global__ void __launch_bounds__(256) k_regress_joints(const float* __restrict_
   }
 }
 
-// one warp per pose, lane = joint (n_joint <= 32)
-__global__ void __launch_bounds__(128) k_normalize_pose2d(const float* __restrict__ px, int batch, int n_joint, int in_h,
-                                                          int in_w, int truncate, float* __restrict__ out) {
-  const int pose = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (pose >= batch) return;
-  const bool on = lane < n_joint;
-  const float x = on ? px[((long long)pose * n_joint + lane) * 2 + 0] : 0.f;
-  const float y = on ? px[((long long)pose * n_joint + lane) * 2 + 1] : 0.f;
+// The box and the affine map of demo/run.py:150-153 for one pose held one joint per lane (all 32 lanes take part;
+// lanes >= n_joint pass on = false): get_bbox, process_bbox(aspect_ratio = width / height, scale), then
+// j2d_processing into a dst_w x dst_h patch.  Returns the processed box [x, y, w, h] and this lane's joint in patch
+// pixels before the reference's cast to float32 (truncated towards zero when truncate is set).
+struct PatchPoint {
+  float box[4];
+  double tx, ty;
+};
+__device__ __forceinline__ PatchPoint pose_to_patch(float x, float y, bool on, float aspect, float scale, int dst_w_px,
+                                                    int dst_h_px, int truncate) {
   float xmin = on ? x : INFINITY, xmax = on ? x : -INFINITY, ymin = on ? y : INFINITY, ymax = on ? y : -INFINITY;
   for (int o = 16; o > 0; o >>= 1) {
     xmin = fminf(xmin, __shfl_xor_sync(0xffffffffu, xmin, o));
@@ -1520,26 +1522,42 @@ __global__ void __launch_bounds__(128) k_normalize_pose2d(const float* __restric
     const double yc = ((double)ymin + (double)ymax) / 2.0, h = (double)ymax - (double)ymin;
     bx = (float)(xc - 0.5 * w); by = (float)(yc - 0.5 * h); bw = (float)w; bh = (float)h;
   }
-  // process_bbox: sanitise (x2 = x + (w - 1)), grow to the aspect ratio width / height, scale 1.0
+  // process_bbox: sanitise (x2 = x + (w - 1)), grow to the aspect ratio width / height, then scale (float32 like numpy
+  // on the float32 box; scale 1.0 leaves the box as it is)
   float w = (bx + (bw - 1.f)) - bx, h = (by + (bh - 1.f)) - by;
   const float cx = bx + w / 2.f, cy = by + h / 2.f;
-  const float aspect = (float)in_w / (float)in_h;
   if (w > aspect * h) h = w / aspect;
   else if (w < aspect * h) w = h * aspect;
+  w = w * scale;
+  h = h * scale;
   const float x0 = cx - w / 2.f, y0 = cy - h / 2.f;
+  PatchPoint p;
+  p.box[0] = x0; p.box[1] = y0; p.box[2] = w; p.box[3] = h;
   // get_center_scale + get_affine_transform(rot = 0): three float32 point pairs, solved in double
   const float ccx = x0 + w * 0.5f, ccy = y0 + h * 0.5f;
   const float s1y = ccy + w * -0.5f;                                     // src[1] = centre + (0, -src_w / 2)
-  const double dst_w = (double)in_w, dst_h = (double)in_h;
+  const double dst_w = (double)dst_w_px, dst_h = (double)dst_h_px;
   const float d1y = (float)(dst_h * 0.5) + (float)(dst_w * -0.5);        // dst[1] = (dst_w / 2, dst_h / 2 - dst_w / 2)
   const double sc = ((double)d1y - dst_h * 0.5) / ((double)s1y - (double)ccy);
-  double tx = ((double)x - (double)ccx) * sc + dst_w * 0.5;
-  double ty = ((double)y - (double)ccy) * sc + dst_h * 0.5;
+  p.tx = ((double)x - (double)ccx) * sc + dst_w * 0.5;
+  p.ty = ((double)y - (double)ccy) * sc + dst_h * 0.5;
   if (truncate) {  // the reference writes the transformed point back into an INTEGER array (demo/h36m_joint_input.npy
-    tx = trunc(tx);  // is int64): truncation towards zero before astype('float32')
-    ty = trunc(ty);
+    p.tx = trunc(p.tx);  // is int64): truncation towards zero before astype('float32')
+    p.ty = trunc(p.ty);
   }
-  float u = (float)tx / (float)in_w, v = (float)ty / (float)in_h;
+  return p;
+}
+
+// one warp per pose, lane = joint (n_joint <= 32)
+__global__ void __launch_bounds__(128) k_normalize_pose2d(const float* __restrict__ px, int batch, int n_joint, int in_h,
+                                                          int in_w, int truncate, float* __restrict__ out) {
+  const int pose = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (pose >= batch) return;
+  const bool on = lane < n_joint;
+  const float x = on ? px[((long long)pose * n_joint + lane) * 2 + 0] : 0.f;
+  const float y = on ? px[((long long)pose * n_joint + lane) * 2 + 1] : 0.f;
+  const PatchPoint p = pose_to_patch(x, y, on, (float)in_w / (float)in_h, 1.f, in_w, in_h, truncate);
+  float u = (float)p.tx / (float)in_w, v = (float)p.ty / (float)in_h;
   // per-pose mean / std (population) per coordinate
   float su = on ? u : 0.f, sv = on ? v : 0.f;
   for (int o = 16; o > 0; o >>= 1) {
@@ -1555,6 +1573,95 @@ __global__ void __launch_bounds__(128) k_normalize_pose2d(const float* __restric
   if (on) {
     out[((long long)pose * n_joint + lane) * 2 + 0] = (u - mu) / sqrtf(qu / n_joint);
     out[((long long)pose * n_joint + lane) * 2 + 1] = (v - mv) / sqrtf(qv / n_joint);
+  }
+}
+
+// The camera fit's projection target (demo/run.py:150-153 with bbox1 = process_bbox(aspect_ratio, scale)): the joints in
+// pixels of the res_w x res_h patch, and the box.  One warp per pose, lane = joint (n_joint <= 32).
+__global__ void __launch_bounds__(128) k_crop_pose2d(const float* __restrict__ px, int batch, int n_joint, int res_w,
+                                                     int res_h, float aspect, float scale, int truncate,
+                                                     float* __restrict__ out, float* __restrict__ out_box) {
+  const int pose = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (pose >= batch) return;
+  const bool on = lane < n_joint;
+  const float x = on ? px[((long long)pose * n_joint + lane) * 2 + 0] : 0.f;
+  const float y = on ? px[((long long)pose * n_joint + lane) * 2 + 1] : 0.f;
+  const PatchPoint p = pose_to_patch(x, y, on, aspect, scale, res_w, res_h, truncate);
+  if (on) {
+    out[((long long)pose * n_joint + lane) * 2 + 0] = (float)p.tx;
+    out[((long long)pose * n_joint + lane) * 2 + 1] = (float)p.ty;
+  }
+  if (lane < 4)  // (a select chain, not p.box[lane]: a lane-dependent index would put the box on the stack)
+    out_box[(long long)pose * 4 + lane] = lane == 0 ? p.box[0] : (lane == 1 ? p.box[1] : (lane == 2 ? p.box[2] : p.box[3]));
+}
+
+// demo/run.py:160-189: the weak-perspective camera of lib/models/project_net.py,
+//   out = (p[:, :2] + c[1:]) * c[0] * R + R,   R = crop_size / 2,
+// fitted to the target by `iters` steps of mean-L1 loss + torch.optim.Adam (defaults, lr 0.1 / 0.05 / 0.001 after steps
+// 501 / 1001).  One warp per person, lane = joint: the camera, the Adam moments and the step count live in registers
+// for the whole fit.  With s = sign(out - tgt) (sign(0) = 0, torch's abs backward) and N = 2 n_joint,
+//   dL/dc1 = R c0 / N * sum_j s_x,   dL/dc2 = R c0 / N * sum_j s_y,   dL/dc0 = R / N * sum_j (s_x a_x + s_y a_y)
+// with a = p + c[1:]: the first two are counts of signs (ballot + popc), the third one float warp reduction.  The
+// arithmetic is written op by op in round-to-nearest (no FMA contraction) in the order of the reference's fp32 torch
+// ops; Adam's bias corrections are computed in double as torch does on the host.
+__device__ __forceinline__ float warp_sum(float v) {
+  // xor butterfly: every lane ends with the same bits (each level adds the same two values, a + b == b + a)
+  for (int o = 16; o > 0; o >>= 1) v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+
+__device__ __forceinline__ void adam_update(float& p, float& m, float& v, float g, float step, float bc2_sqrt) {
+  m = __fadd_rn(m, __fmul_rn(0.1f, __fsub_rn(g, m)));                       // exp_avg.lerp_(grad, 1 - beta1)
+  v = __fadd_rn(__fmul_rn(v, 0.999f), __fmul_rn(__fmul_rn(0.001f, g), g));  // exp_avg_sq.mul_(b2).addcmul_(g, g, 1 - b2)
+  const float denom = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), bc2_sqrt), 1e-8f);
+  p = __fadd_rn(p, __fdiv_rn(__fmul_rn(-step, m), denom));                  // param.addcdiv_(m, denom, -step_size)
+}
+
+__global__ void __launch_bounds__(128) k_fit_camera(const float* __restrict__ j3d, const float* __restrict__ tgt,
+                                                    const float* __restrict__ cam_init, int batch, int n_joint,
+                                                    int stride, float R, int iters, float* __restrict__ cam_out,
+                                                    float* __restrict__ loss_out) {
+  const int b = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= batch) return;
+  const bool on = lane < n_joint;
+  const long long jb = (long long)b * n_joint + lane;
+  const float px = on ? j3d[jb * stride + 0] : 0.f, py = on ? j3d[jb * stride + 1] : 0.f;
+  const float qx = on ? tgt[jb * 2 + 0] : 0.f, qy = on ? tgt[jb * 2 + 1] : 0.f;
+  float c0 = cam_init[b * 3 + 0], c1 = cam_init[b * 3 + 1], c2 = cam_init[b * 3 + 2];
+  float m0 = 0.f, m1 = 0.f, m2 = 0.f, v0 = 0.f, v1 = 0.f, v2 = 0.f;
+  const float gs = __fmul_rn(__fdiv_rn(1.f, (float)(2 * n_joint)), R);  // mean backward (1 / N), then the "* R"
+  for (int t = 1; t <= iters; ++t) {
+    const float ax = __fadd_rn(px, c1), ay = __fadd_rn(py, c2);
+    const float rx = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(ax, c0), R), R), qx);
+    const float ry = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(ay, c0), R), R), qy);
+    const int sx = __popc(__ballot_sync(0xffffffffu, on && rx > 0.f)) - __popc(__ballot_sync(0xffffffffu, on && rx < 0.f));
+    const int sy = __popc(__ballot_sync(0xffffffffu, on && ry > 0.f)) - __popc(__ballot_sync(0xffffffffu, on && ry < 0.f));
+    float sa = 0.f;
+    if (on) {
+      sa = rx > 0.f ? ax : (rx < 0.f ? -ax : 0.f);
+      sa = __fadd_rn(sa, ry > 0.f ? ay : (ry < 0.f ? -ay : 0.f));
+    }
+    const float g0 = __fmul_rn(gs, warp_sum(sa));
+    const float gc = __fmul_rn(gs, c0);
+    const float g1 = __fmul_rn((float)sx, gc), g2 = __fmul_rn((float)sy, gc);
+    // lr schedule of run.py:181-186 (the change after loop index 500 / 1000 applies from the next step on)
+    const double lr = t <= 501 ? 0.1 : (t <= 1001 ? 0.05 : 0.001);
+    const float step = (float)(lr / (1.0 - pow(0.9, (double)t)));
+    const float bc2_sqrt = (float)sqrt(1.0 - pow(0.999, (double)t));
+    adam_update(c0, m0, v0, g0, step, bc2_sqrt);
+    adam_update(c1, m1, v1, g1, step, bc2_sqrt);
+    adam_update(c2, m2, v2, g2, step, bc2_sqrt);
+  }
+  // L1 loss of the final camera (nn.L1Loss: mean over the n_joint x 2 residuals)
+  const float ax = __fadd_rn(px, c1), ay = __fadd_rn(py, c2);
+  const float rx = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(ax, c0), R), R), qx);
+  const float ry = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(ay, c0), R), R), qy);
+  const float l = warp_sum(on ? __fadd_rn(fabsf(rx), fabsf(ry)) : 0.f);
+  if (lane == 0) {
+    cam_out[b * 3 + 0] = c0;
+    cam_out[b * 3 + 1] = c1;
+    cam_out[b * 3 + 2] = c2;
+    loss_out[b] = __fdiv_rn(l, (float)(2 * n_joint));
   }
 }
 }  // namespace
@@ -1582,6 +1689,41 @@ int p2m_normalize_pose2d(const float* joints_px, float* pose2d, int batch, int n
   }
   k_normalize_pose2d<<<(batch + 3) / 4, 128, 0, static_cast<cudaStream_t>(stream)>>>(joints_px, batch, n_joint, input_h,
                                                                                    input_w, truncate_like_int_input, pose2d);
+  P2M_LAUNCH_OK();
+  return P2M_OK;
+}
+
+int p2m_crop_pose2d(const float* joints_px, float* out_px, float* out_bbox, int batch, int n_joint, int res_w, int res_h,
+                    float aspect_ratio, float scale, int truncate_like_int_input, p2m_stream_t stream) {
+  if (!joints_px || !out_px || !out_bbox || batch <= 0 || n_joint <= 0 || n_joint > 32 || res_w <= 0 || res_h <= 0 ||
+      !(aspect_ratio > 0.f) || !(scale > 0.f)) {
+    set_error("crop_pose2d: bad argument (null pointer, at most 32 joints, positive patch size / aspect ratio / scale)");
+    return P2M_ERR_INVALID;
+  }
+  k_crop_pose2d<<<(batch + 3) / 4, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      joints_px, batch, n_joint, res_w, res_h, aspect_ratio, scale, truncate_like_int_input, out_px, out_bbox);
+  P2M_LAUNCH_OK();
+  return P2M_OK;
+}
+
+int p2m_fit_camera(const float* joints3d, const float* target_px, const float* cam_init, float* cam_out, float* loss_out,
+                   int batch, int n_joint, int joint_stride, double crop_size, int iters, p2m_stream_t stream) {
+  if (!joints3d || !target_px || !cam_init || !cam_out || !loss_out) {
+    set_error("fit_camera: null pointer");
+    return P2M_ERR_INVALID;
+  }
+  if (batch <= 0 || n_joint <= 0 || n_joint > 32) {
+    set_error("fit_camera: need batch >= 1 and 1 <= n_joint <= 32 (got batch " + std::to_string(batch) + ", n_joint " +
+              std::to_string(n_joint) + ")");
+    return P2M_ERR_INVALID;
+  }
+  if (joint_stride < 2 || iters < 1 || !(crop_size > 0.0)) {
+    set_error("fit_camera: need joint_stride >= 2, iters >= 1 and crop_size > 0 (got " + std::to_string(joint_stride) +
+              ", " + std::to_string(iters) + ", " + std::to_string(crop_size) + ")");
+    return P2M_ERR_INVALID;
+  }
+  k_fit_camera<<<(batch + 3) / 4, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      joints3d, target_px, cam_init, batch, n_joint, joint_stride, (float)(crop_size / 2.0), iters, cam_out, loss_out);
   P2M_LAUNCH_OK();
   return P2M_OK;
 }

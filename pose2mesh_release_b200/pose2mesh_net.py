@@ -47,6 +47,39 @@ class FlatPose2Mesh(nn.Module):
         joints = postprocess.regress_joints(verts, joint_regressor)
         return verts, joints, pose3d.reshape(-1, self.num_joint, 3)
 
+    @torch.no_grad()
+    def optimize_cam_param(self, joints_px, perm_reverse, n_vertex, joint_regressor, crop_size=500, cam_init=None):
+        """demo/run.py:149-197 for B people in one call: joints_px [B, J_in, 2 | 3] image pixels (an integer tensor is
+        truncated like the demo's int64 input; a third column is ignored) -> dict of the demo's ``out`` fields,
+        batched: ``mesh`` [B, n_vertex, 3], ``cam_param`` [B, 3], ``bbox`` [B, 4] (bbox1), ``target`` [B, J_in, 2],
+        plus ``loss`` [B], the L1 loss of each fitted camera.
+
+        Chains normalize_pose2d -> predict_vertices_and_joints -> crop_pose2d -> fit_camera.  Like the demo, the fit
+        pairs the regressed joints with the first 17 target joints (run.py:180), so joint_regressor must have 17 rows.
+        cam_init=None draws torch.rand((1, 3)) once per person, in order, as the demo's per-person
+        project_net.get_model does."""
+        from . import project_net
+
+        dev = next(self.parameters()).device
+        jp = torch.as_tensor(joints_px)
+        if jp.dim() == 2:
+            jp = jp[None]
+        if jp.dim() != 3 or jp.shape[2] not in (2, 3):
+            raise ValueError(f"joints_px must be [B, J, 2 | 3], got {tuple(jp.shape)}")
+        n_reg = joint_regressor.shape[0]
+        if n_reg != 17 or jp.shape[1] < 17:
+            raise ValueError(f"the demo's camera fit pairs 17 regressed joints with the first 17 input joints "
+                             f"(demo/run.py:180); got a {n_reg}-row joint_regressor and {jp.shape[1]} input joints")
+        B = jp.shape[0]
+        if cam_init is None:
+            cam_init = torch.cat([torch.rand((1, 3)) for _ in range(B)])
+        jp = jp[..., :2].to(dev)
+        pose2d = postprocess.normalize_pose2d(jp)
+        verts, joints, _ = self.predict_vertices_and_joints(pose2d, perm_reverse, n_vertex, joint_regressor)
+        target, bbox = postprocess.crop_pose2d(jp, res=crop_size, aspect_ratio=1.0, scale=1.25)
+        cam, loss = project_net.fit_camera(joints, target[:, :17].contiguous(), crop_size, cam_init.to(dev))
+        return {"mesh": verts, "cam_param": cam, "bbox": bbox, "target": target, "loss": loss}
+
 
 def get_model(num_joint, graph_L):
     """lib/models/pose2mesh_net.py:25-28."""
